@@ -26,6 +26,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree it runs from as it found it (which may be read-only)
 
 from loam_livox_b200 import synthetic as S  # noqa: E402
 
@@ -266,6 +267,22 @@ def check_against_oracle(step, inputs, world_note=""):
     return worst_t, worst_a
 
 
+def dump_outputs(out_dir, ctx, res, nc, ns):
+    """What the caller of ll_scan_to_pose receives from the last timed step (pose, increment, costs and counts of the ll_reg_result, feature counts),
+    plus the scan-frame feature clouds that registration matched (x, y, z, intensity), one DIR/<name>.npy each.  The inputs are seeded, so two
+    builds run with the same arguments can be compared file by file."""
+    from loam_livox_b200.registration import features_to_pointcloud2
+    out = {"q_w_curr": np.array(res.q_w_curr), "t_w_curr": np.array(res.t_w_curr), "q_w_incre": np.array(res.q_w_incre), "t_w_incre": np.array(res.t_w_incre),
+           "costs": np.array([res.initial_cost, res.final_cost, res.inlier_threshold, res.angular_diff, res.t_diff]),
+           "counts": np.array([res.status, res.registered, res.num_residual_blocks, res.icp_iterations, res.corner_used, res.surf_used,
+                               res.total_lm_iterations, res.total_evaluations, nc, ns], np.float64),
+           "corner_features": np.frombuffer(features_to_pointcloud2(ctx, 0), np.float32).reshape(-1, 4),
+           "surface_features": np.frombuffer(features_to_pointcloud2(ctx, 1), np.float32).reshape(-1, 4)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_gpu(args):
     import ctypes as C
     import torch
@@ -378,6 +395,7 @@ def run_gpu(args):
             note(res, nc, ns)
         torch.cuda.synchronize()
         total_ms = float(np.sum([a.elapsed_time(b) for a, b in ev]))
+        last, last_ctx = (res, nc, ns), ctx
     else:
         # throughput mode: K host threads, one context each, all on the shared map; the device time is the span from the first start event to the
         # last end event (events of different streams of one device share a clock); the L2 cannot be flushed between steps of concurrent streams,
@@ -407,7 +425,11 @@ def run_gpu(args):
         for r in results:
             for (res, nc, ns) in r:
                 note(res, nc, ns)
+        w = (args.steps - 1) % K
+        last, last_ctx = results[w][-1], ctxs[w]
     launches = sum(c.launches() for c in ctxs) - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_ctx, *last)
     # ---- e2e: pinned host inputs through the same public call, host wall clock, H2D + result D2H inside
     if K == 1:
         e2e_s = 0.0
@@ -691,7 +713,11 @@ def main():
     ap.add_argument("--dump-poses", default=None, help="c3 only: write the pose after every scan (q_wxyz, t) to this .npy (diagnostics: first scan at which GPU and oracle part)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--cpu-scans", type=int, default=5)
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR", help="--workload c2 (either --mode) only: after the timed steps, write what "
+                    "the last one returned (pose, increment, costs, counts, feature clouds) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.workload != "c2"):
+        ap.error("--dump-outputs writes the outputs of the GPU registration path (--impl ours, --workload c2)")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

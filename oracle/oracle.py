@@ -84,7 +84,8 @@ def default_params(**kw) -> RegParams:
 def build(force: bool = False) -> str:
     so = os.path.join(_HERE, "liboracle.so")
     srcs = [os.path.join(_HERE, f) for f in os.listdir(_HERE) if f.endswith((".cpp", ".hpp"))]
-    if force or not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in srcs):
+    # a read-only tree (a built checkout the benchmark runs from) keeps the library it was built with
+    if force or not os.path.exists(so) or (os.access(_HERE, os.W_OK) and any(os.path.getmtime(s) > os.path.getmtime(so) for s in srcs)):
         subprocess.check_call(["make", "-C", _HERE, "-s"])
     return so
 
