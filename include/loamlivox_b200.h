@@ -185,6 +185,14 @@ int ll_register(ll_ctx* ctx, const ll_map* map, const void* scan_corner, size_t 
  * (type 0 invalid / 1 line / 2 plane, a[3], v[3] per slot; slots = corner features then surface features) ... */
 int ll_build_blocks(ll_ctx* ctx, const ll_map* map, const void* scan_corner, size_t n_corner, const void* scan_surf, size_t n_surf,
                     int fmt, int where, const ll_reg_state* in, int32_t* type, double* a3, double* v3, int* corner_avail, int* surf_avail);
+/* ... and the same launch as one ICP iteration of ll_register runs it (the kNN kernel variant the context selected, LL_KNN_TMA=1 at
+ * ll_ctx_create), at ICP iteration icp_iter (the residual-block cap's pre-skip draws) and with caller-chosen seeds: seeds_in [M x 5] are the
+ * neighbour ids a search starts from (-1 = none; NULL = all -1), as the previous ICP iteration leaves them.  Out: idx5 / d5 [M x 5] the
+ * neighbour ids (-1 when fewer exist) and fp32 squared distances, type / a3 / v3 the slots as ll_build_blocks, *tma_variant = 1 when the
+ * TMA-staged kernel ran.  A row the kernel leaves inactive (pre-skipped, non-finite or not owned) keeps its input seeds, with NaN distances. */
+int ll_debug_knn_blocks(ll_ctx* ctx, const ll_map* map, const void* scan_corner, size_t n_corner, const void* scan_surf, size_t n_surf, int fmt, int where,
+                        const ll_reg_state* in, int icp_iter, const int32_t* seeds_in, int32_t* idx5, float* d5, int32_t* type, double* a3, double* v3,
+                        int* tma_variant);
 /* ... and the loss-corrected normal equations at x (q x,y,z,w ; t): out28 = 21 upper-triangular JtJ (row-major), 6 Jtr, cost. */
 int ll_normal_equations(ll_ctx* ctx, const double x[7], double out28[28]);
 /* ... and one ceres::Solve-equivalent on the blocks currently resident (max_iterations as in Solver::Options). */

@@ -23,7 +23,7 @@ EXPORTS = [
     "ll_config_default", "ll_ctx_create", "ll_ctx_destroy", "ll_ctx_warmup", "ll_last_error", "ll_ctx_stream", "ll_ctx_sync", "ll_extract", "ll_extract_reset", "ll_piece_bounds",
     "ll_get_features", "ll_extract_point_info", "ll_extract_split_idx", "ll_voxel_downsample", "ll_map_build", "ll_map_release", "ll_map_size",
     "ll_map_build_sharded", "ll_knn", "ll_reg_state_default", "ll_register", "ll_build_blocks", "ll_normal_equations", "ll_solve", "ll_transform",
-    "ll_scan_to_pose", "ll_comm_local_handle", "ll_comm_connect", "ll_launch_count", "ll_cellmap_create", "ll_cellmap_release", "ll_cellmap_append",
+    "ll_debug_knn_blocks", "ll_scan_to_pose", "ll_comm_local_handle", "ll_comm_connect", "ll_launch_count", "ll_cellmap_create", "ll_cellmap_release", "ll_cellmap_append",
     "ll_cellmap_assemble", "ll_cellmap_reserve", "ll_cellmap_stats", "ll_voxel_downsample_dev", "ll_transform_dev", "ll_last_features_dev", "ll_mapper_config_default", "ll_mapper_create", "ll_mapper_release",
     "ll_mapper_process_scan", "ll_mapper_pose", "ll_map_rebuild", "ll_debug_solver_cycles", "ll_state_snapshot_bytes", "ll_set_point_layout", "ll_format_pose_log", "ll_reg_state_yaml", "ll_cap_uniform", "ll_map_shard_info", "ll_shard_plan", "ll_align_cfg_default", "ll_scene_align", "ll_frame_to_pose", "ll_features_to_pointcloud2",
 ]
@@ -132,6 +132,7 @@ def lib():
     L.ll_cap_uniform.restype = cf
     L.ll_register.argtypes = [vp, vp, vp, sz, vp, sz, ci, ci, C.POINTER(RegState), C.POINTER(RegResult)]
     L.ll_build_blocks.argtypes = [vp, vp, vp, sz, vp, sz, ci, ci, C.POINTER(RegState), vp, vp, vp, C.POINTER(ci), C.POINTER(ci)]
+    L.ll_debug_knn_blocks.argtypes = [vp, vp, vp, sz, vp, sz, ci, ci, C.POINTER(RegState), ci, vp, vp, vp, vp, vp, vp, C.POINTER(ci)]
     L.ll_normal_equations.argtypes = [vp, vp, vp]
     L.ll_solve.argtypes = [vp, ci, vp, C.POINTER(cd), C.POINTER(cd), C.POINTER(ci)]
     L.ll_transform.argtypes = [vp, vp, vp, vp, sz, ci, ci, vp]

@@ -517,8 +517,10 @@ int ll_ctx_warmup(ll_ctx* ctx) {
   return st;
 }
 
-int ll_build_blocks(ll_ctx* ctx, const ll_map* map, const void* scan_corner, size_t nc, const void* scan_surf, size_t ns, int fmt, int where, const ll_reg_state* in,
-                    int32_t* type, double* a3, double* v3, int* corner_avail, int* surf_avail) {
+// One ICP iteration's kNN + residual-block launch at the pose in `in`, ICP iteration icp_iter, seeded with seeds_in ([M x 5], NULL = no seeds),
+// followed by the read-back of the slots; idx5 / d5 (may be NULL) receive the search's neighbour ids and squared distances.
+static int blocks_hook(ll_ctx* ctx, const ll_map* map, const void* scan_corner, size_t nc, const void* scan_surf, size_t ns, int fmt, int where, const ll_reg_state* in,
+                       int icp_iter, const int32_t* seeds_in, int32_t* idx5, float* d5, int32_t* type, double* a3, double* v3, int* corner_avail, int* surf_avail) {
   if (!ctx || !map || !in) return LL_ERR_INVALID;
   cudaSetDevice(ctx->device);
   const int M = (int)(nc + ns);
@@ -528,13 +530,20 @@ int ll_build_blocks(ll_ctx* ctx, const ll_map* map, const void* scan_corner, siz
   LL_TRY(upload_cloud(ctx, scan_corner, nc, fmt, where, A.feat));
   LL_TRY(upload_cloud(ctx, scan_surf, ns, fmt, where, A.feat + nc));
   RegDevState* h = (RegDevState*)ctx->pinned; fill_state(h, in);
+  h->icp_iter = icp_iter;   // the cap's pre-skip draws depend on the ICP iteration
   LL_CUDA(ctx, cudaMemcpyAsync(ctx->d_reg, h, sizeof(RegDevState), cudaMemcpyHostToDevice, s));
-  { KnnBlocksArgs ka = knn_args(ctx, map, A, (int)nc, (int)ns, in, true); LL_CUDA(ctx, cudaMemsetAsync(A.knn_idx, 0xff, (size_t)M * LL_KNN * 4, s)); LL_TRY(launch_query_sort(ctx, ka, A.perm)); LL_TRY(launch_knn_blocks(ctx, ka)); }
+  const size_t row_bytes = (size_t)M * LL_KNN * 4;
+  if (seeds_in) { if (M > 0) LL_CUDA(ctx, cudaMemcpyAsync(A.knn_idx, seeds_in, row_bytes, cudaMemcpyHostToDevice, s)); }
+  else LL_CUDA(ctx, cudaMemsetAsync(A.knn_idx, 0xff, row_bytes, s));
+  LL_CUDA(ctx, cudaMemsetAsync(A.knn_d, 0xff, row_bytes, s));   // NaN: rows the kernel leaves inactive keep it
+  { KnnBlocksArgs ka = knn_args(ctx, map, A, (int)nc, (int)ns, in, true); LL_TRY(launch_query_sort(ctx, ka, A.perm)); LL_TRY(launch_knn_blocks(ctx, ka)); }
   std::vector<float4> ba(M); std::vector<double> bv((size_t)M * 3);
   int cnt[2];
   LL_CUDA(ctx, cudaMemcpyAsync(ba.data(), A.blk_a, (size_t)M * 16, cudaMemcpyDeviceToHost, s));
   LL_CUDA(ctx, cudaMemcpyAsync(bv.data(), A.blk_v, (size_t)M * 24, cudaMemcpyDeviceToHost, s));
   LL_CUDA(ctx, cudaMemcpyAsync(cnt, &ctx->d_reg->corner_avail, 8, cudaMemcpyDeviceToHost, s));
+  if (idx5 && M > 0) LL_CUDA(ctx, cudaMemcpyAsync(idx5, A.knn_idx, row_bytes, cudaMemcpyDeviceToHost, s));
+  if (d5 && M > 0) LL_CUDA(ctx, cudaMemcpyAsync(d5, A.knn_d, row_bytes, cudaMemcpyDeviceToHost, s));
   LL_CUDA(ctx, cudaStreamSynchronize(s));
   for (int i = 0; i < M; i++) {
     int t; memcpy(&t, &ba[i].w, 4);
@@ -545,6 +554,17 @@ int ll_build_blocks(ll_ctx* ctx, const ll_map* map, const void* scan_corner, siz
   if (corner_avail) *corner_avail = cnt[0]; if (surf_avail) *surf_avail = cnt[1];
   ctx->hook_slots = M;   // slot count for ll_normal_equations / ll_solve
   return LL_OK;
+}
+int ll_build_blocks(ll_ctx* ctx, const ll_map* map, const void* scan_corner, size_t nc, const void* scan_surf, size_t ns, int fmt, int where, const ll_reg_state* in,
+                    int32_t* type, double* a3, double* v3, int* corner_avail, int* surf_avail) {
+  return blocks_hook(ctx, map, scan_corner, nc, scan_surf, ns, fmt, where, in, 0, nullptr, nullptr, nullptr, type, a3, v3, corner_avail, surf_avail);
+}
+int ll_debug_knn_blocks(ll_ctx* ctx, const ll_map* map, const void* scan_corner, size_t nc, const void* scan_surf, size_t ns, int fmt, int where,
+                        const ll_reg_state* in, int icp_iter, const int32_t* seeds_in, int32_t* idx5, float* d5, int32_t* type, double* a3, double* v3,
+                        int* tma_variant) {
+  const int st = blocks_hook(ctx, map, scan_corner, nc, scan_surf, ns, fmt, where, in, icp_iter, seeds_in, idx5, d5, type, a3, v3, nullptr, nullptr);
+  if (st == LL_OK && tma_variant) *tma_variant = ctx->knn_tma;
+  return st;
 }
 int ll_normal_equations(ll_ctx* ctx, const double x[7], double out28[28]) {
   if (!ctx || !x || !out28) return LL_ERR_INVALID;

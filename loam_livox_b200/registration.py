@@ -236,6 +236,28 @@ class Point_cloud_registration:
                                                      typ.ctypes.data, a3.ctypes.data, v3.ctypes.data, C.byref(ca), C.byref(sa)))
         return typ, a3, v3, ca.value, sa.value
 
+    def debug_knn_blocks(self, match_map: Map, corner, surf, icp_iter: int = 0, seeds=None):
+        """One ICP iteration's kNN + residual-block launch as ll_register runs it (the context's kernel variant), at ICP iteration icp_iter and
+        with seeds [M,5] int32 (-1 = none; None = no seeds).  Returns (idx5 [M,5] int32, d5 [M,5] float32, type, a3, v3, tma_variant); a row the
+        kernel leaves inactive keeps its seeds, with NaN distances."""
+        c, fmt = _pts(corner)
+        s, _ = _pts(surf)
+        M = c.shape[0] + s.shape[0]
+        sd = None
+        if seeds is not None:
+            sd = np.ascontiguousarray(seeds, np.int32)
+            assert sd.shape == (M, 5)
+        idx = np.empty((M, 5), np.int32)
+        d2 = np.empty((M, 5), np.float32)
+        typ = np.zeros(M, np.int32)
+        a3 = np.zeros((M, 3))
+        v3 = np.zeros((M, 3))
+        tma = C.c_int(-1)
+        self.ctx.check(self.ctx._lib.ll_debug_knn_blocks(self.ctx.h, match_map.h, c.ctypes.data, c.shape[0], s.ctypes.data, s.shape[0], fmt, capi.LL_HOST,
+                                                         C.byref(self.state), int(icp_iter), None if sd is None else sd.ctypes.data, idx.ctypes.data,
+                                                         d2.ctypes.data, typ.ctypes.data, a3.ctypes.data, v3.ctypes.data, C.byref(tma)))
+        return idx, d2, typ, a3, v3, tma.value
+
     def normal_equations(self, x7):
         x = np.ascontiguousarray(x7, np.float64)
         out = np.zeros(28)
